@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the B200-native MegReader recognition hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): CRNN backbone + 2x BiLSTM + 1D CTC, synthetic 32x256 lines (gray replicated to
 3 channels, SURVEY.md D2), batch 512 PER GPU (weak scaling), bf16 compute, one full training step per "step":
@@ -13,6 +13,11 @@ Prints ONE JSON line (rank 0).  Extra objects on that line:
   roofline     the dominant hand-written kernel, algorithmic bytes / CUDA-event time vs MEASURED_PEAKS.json
   ctc2d        second half of BASELINE.json's metric: 2D-CTC fwd+bwd GB/s at the cfg-3 shape, saturating batch
   cpu_baseline the oracle port of the same step timed on this box's host cores (bounded sample)
+--dump-outputs DIR writes what the last timed step returned (rank 0), its loss and log-probabilities, as DIR/<name>.npy in
+float32.  That step starts from the seeded initial parameters, which are put back just before it: the steps before it train
+with split-K atomic weight gradients whose summation order varies from run to run, and Adam would carry that into the
+parameters.  Its inputs therefore depend on the arguments only, and two builds run with the same arguments can be compared
+output for output.
 --impl reference runs only the CPU arm (oracle port = restatement of the reference's own CPU path; the python
 reference itself cannot travel to the GPU box) and prints the same line shape with "impl": "reference".
 """
@@ -142,6 +147,7 @@ def run_ours(args):
     net = build_model(dev)
     model = net
     params = list(net.parameters())
+    initial = [p.detach().clone() for p in params] if args.dump_outputs else None
     opt = torch.optim.Adam(params, lr=1e-3, fused=True, capturable=True)   # optimizer_scheduler.py:17-22, lr crnn.yaml
     from megreader_b200 import crnn_engine, dp
     crnn_engine.set_compute_dtype(torch.bfloat16)          # BASELINE.json cfg 2: bf16 compute, fp32 master weights
@@ -163,12 +169,12 @@ def run_ours(args):
             fg.zero()                                      # one memset; the .grad views stay attached
         else:
             opt.zero_grad(set_to_none=True)
-        loss, _ = model(x, y, l)
+        loss, pred = model(x, y, l)
         loss.mean().backward()
-        return loss
+        return loss, pred
 
     def eager_step(x, y, l):
-        loss = fwd_bwd(x, y, l)
+        loss, _ = fwd_bwd(x, y, l)
         if fg is not None:
             fg.allreduce_()                                # NCCL all-reduce(AVG), in place on the flat 33 MB buffer
         opt.step()
@@ -197,7 +203,7 @@ def run_ours(args):
     _lib.reset_launch_count()
     graph_a = torch.cuda.CUDAGraph()
     with torch.cuda.graph(graph_a):
-        static_loss = fwd_bwd(*static)
+        static_loss, static_pred = fwd_bwd(*static)
         if world == 1:
             opt.step()
     graph_b = None
@@ -226,13 +232,23 @@ def run_ours(args):
     if sampler:
         sampler.start()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    reset = None                                           # events around the parameter reset: its time is not step time
     e0.record()
     for i in range(args.steps):
+        if initial is not None and i == args.steps - 1:
+            reset = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            reset[0].record()
+            with torch.no_grad():
+                for p, p0 in zip(params, initial):
+                    p.copy_(p0)
+            reset[1].record()
         loss = step(*dev_batches[i % n_host])
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"loss": static_loss, "log_probs": static_pred})
     launches = launches_per_step * args.steps          # kernels of this library inside the replayed graphs
-    ms = e0.elapsed_time(e1)
+    ms = e0.elapsed_time(e1) - (reset[0].elapsed_time(reset[1]) if reset else 0.0)
     clocks = sampler.stop() if sampler else None
     final_loss = float(loss.mean().item())
 
@@ -284,6 +300,10 @@ def run_ours(args):
                 "ms_per_step": ms_e2e / args.steps},
         "gpu_launches": launches, "final_loss": final_loss, "clocks": clocks,
     }
+    if args.dump_outputs:
+        out["dump_outputs"] = {"dir": args.dump_outputs, "files": ["loss.npy", "log_probs.npy"],
+                               "last_step": "started from the seeded initial parameters (the reset before it is excluded from "
+                                            "ms_per_step); final_loss is that step's loss"}
     if crnn_engine.LAST_LSTM_FLAGS is not None:            # error word of the persistent LSTM kernels (0 = no wait timed out)
         out["lstm_seq_err"] = int(crnn_engine.LAST_LSTM_FLAGS[-1])
         if out["lstm_seq_err"]:
@@ -324,6 +344,19 @@ def run_ours(args):
         emit_json(out)
     if world > 1:
         dist.destroy_process_group()
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> device tensor, written as path/<name>.npy in float32 (at most DUMP_LIMIT bytes in all)"""
+    total = sum(t.numel() * 4 for t in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------- 2D-CTC micro arm
@@ -592,7 +625,8 @@ def usable_cores():
 
 def cpu_arm(steps, warmup, sample_n, budget_s=25.0):
     """The reference's own CPU path for this workload, restated by oracle/crnn_port.py (validated bit-for-bit against
-    the unmodified reference modules in the build container): fp32, all host cores, same model/optimizer."""
+    the unmodified reference modules in the build container): fp32, all host cores, same model/optimizer.  With a budget
+    (seconds) the warm-up stops after half of it and the timed steps after all of it; budget_s=None runs every step."""
     from oracle import crnn_port
     from tests.weights import fill_state_dict
     cores = usable_cores()
@@ -611,14 +645,14 @@ def cpu_arm(steps, warmup, sample_n, budget_s=25.0):
     tw = time.perf_counter()
     for _ in range(warmup):
         step()
-        if time.perf_counter() - tw > budget_s / 2:
+        if budget_s is not None and time.perf_counter() - tw > budget_s / 2:
             break
     t0 = time.perf_counter()
     done = 0
     for _ in range(steps):
         step()
         done += 1
-        if time.perf_counter() - t0 > budget_s:
+        if budget_s is not None and time.perf_counter() - t0 > budget_s:
             break
     steps = done
     dt = time.perf_counter() - t0
@@ -690,7 +724,7 @@ def run_reference(args):
     if rank != 0:
         return
     n = 32
-    res = cpu_arm(steps=args.steps, warmup=args.warmup, sample_n=n)
+    res = cpu_arm(steps=args.steps, warmup=args.warmup, sample_n=n, budget_s=None)     # --steps is the number of timed steps
     out = {"impl": "reference", "metric": METRIC, "value": res["value"], "unit": "lines/s", "n_gpus": args.gpus,
            "steps": args.steps, "warmup": args.warmup, "ms_per_step": res["ms_per_step"],
            "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -739,10 +773,17 @@ def main():
                     help="BASELINE.json configuration: 2 = CRNN + 1D CTC (headline, default); 3 = ResNet50-PPM + 2D CTC; "
                          "4 = FPN50 + attention decoder; 5 = deformable ResNet50 + FPN + EAST (bench_trunks.py)")
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch for --config 3 / 4 (default 32)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's loss and log-probabilities as DIR/<name>.npy; that "
+                         "step starts from the seeded initial parameters (headline workload only)")
     ap.add_argument("--strong", action="store_true",
                     help="reference semantics (data/data_loader.py:40-43): global batch 512 split over the ranks (strong scaling) "
                          "instead of 512 per GPU")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != 2):
+        ap.error("--dump-outputs is implemented for the headline workload (--impl ours --config 2)")
     if args.impl == "reference":
         run_reference(args)
     elif args.config != 2:

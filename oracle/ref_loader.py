@@ -1,10 +1,8 @@
-"""Import the UNMODIFIED reference modules from /root/reference (build container only).
+"""Import the UNMODIFIED reference modules from the reference checkout (MEGREADER_REFERENCE).
 
 The reference's third-party deps (tensorboardX, apex, anyconfig, ...) are not installed, so
-stub modules are injected into sys.modules first.  /root/reference does not exist on the GPU
-box: nothing under tests/ -m gpu, smoke() or bench.py imports this file at run time; it is used
-only by oracle/make_golden.py to generate tests/golden/*.npz (committed), and by `-m "not gpu"`
-tests that skip when the reference is absent.
+stub modules are injected into sys.modules first.  Only oracle/make_golden.py imports this
+file, to record tests/golden/* (committed): no test, smoke() or bench.py needs the reference.
 """
 import importlib
 import os

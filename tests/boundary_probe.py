@@ -1,50 +1,41 @@
-"""Helper of tests/test_boundary_yaml_cpu.py (run as a subprocess): build the models of the reference's three recognition yamls with the
-reference's OWN structure/model.py and concern/charsets.py, with `backbones` / `decoders` / `ops` / `assets` resolved either to the
-reference (mode "reference") or to megreader_b200/refapi (mode "refapi").  Prints one JSON object."""
+"""Helper of tests/test_boundary_yaml_cpu.py (run as a subprocess, so that the reference's top-level names stay out of the test
+process): build the models of the reference's three recognition yamls from their recorded `model_args`, with `backbones` /
+`decoders` / `ops` / `assets` resolved to megreader_b200/refapi, composed as structure/model.py:16-24 BasicModel composes them.
+Prints one JSON object."""
+import gzip
 import json
 import os
 import sys
-import types
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-mode = sys.argv[1]
-from oracle import ref_loader  # noqa: E402
+import megreader_b200  # noqa: E402
+from megreader_b200 import charset as mcharset  # noqa: E402
 
-assert ref_loader.install()
-REF = ref_loader.REF
-if mode == "refapi":
-    import megreader_b200
-    refapi_dir = os.path.join(os.path.dirname(megreader_b200.__file__), "refapi")
-    sys.path.insert(0, refapi_dir)                       # ahead of the reference: backbones / decoders / ops / assets are ours
-else:
-    # the reference's native 2D-CTC extension is not built for CPU: its import site only needs the module object
-    for name in ("ops.ctc_2d.ctc_2d_csrc",):
-        sys.modules[name] = types.ModuleType(name)
+sys.path.insert(0, os.path.join(os.path.dirname(megreader_b200.__file__), "refapi"))
 import torch  # noqa: E402
-import yaml  # noqa: E402
 import backbones  # noqa: E402
 import decoders  # noqa: E402
-import structure.model as smodel  # noqa: E402  (always the reference's file)
-import concern.charsets as charsets  # noqa: E402
 
-assert smodel.__file__.startswith(REF) and charsets.__file__.startswith(REF)
-out = {"backbones_file": backbones.__file__, "decoders_file": decoders.__file__, "models": {}}
-base = yaml.safe_load(open(os.path.join(REF, "experiments/recognition/community-base.yaml")))
-cs_def = [d for d in base["define"] if d["name"] == "charset"][0]
-charset = getattr(charsets, cs_def["class"])()
-for y in ("crnn.yaml", "res50-ppm-2d-ctc.yaml", "fpn50-attention-decoder.yaml"):
-    conf = yaml.safe_load(open(os.path.join(REF, "experiments/recognition", y)))
-    st = [d for d in conf["define"] if d["name"] == "BasicStructure"][0]
-    builder = st["builder"]
-    args = json.loads(json.dumps(builder["model_args"]))
+
+class BasicModel(torch.nn.Module):
+    def __init__(self, args):
+        super().__init__()
+        self.backbone = getattr(backbones, args["backbone"])(**args.get("backbone_args", {}))
+        self.decoder = getattr(decoders, args["decoder"])(**args.get("decoder_args", {}))
+
+
+with gzip.open(os.path.join(ROOT, "tests", "golden", "state_dicts_ref.json.gz"), "rt") as f:
+    gold = json.load(f)
+charset = getattr(mcharset, gold["charset"]["class"])()
+out = {"backbones_file": backbones.__file__, "decoders_file": decoders.__file__, "charset_len": len(charset), "models": {}}
+for y, rec in gold["yamls"].items():
+    args = json.loads(json.dumps(rec["model_args"]))
     for k, v in list(args.get("decoder_args", {}).items()):
         if v == "^charset":
             args["decoder_args"][k] = charset
-    if "resnet" in args["backbone"].lower():
-        args.setdefault("backbone_args", {})["resnet_pretrained"] = False      # no network for the torchvision checkpoint
-    model = getattr(smodel, builder["model"])(args, torch.device("cpu"))      # structure/model.py:160-166 -> BasicModel :16-24
-    out["models"][y] = {"model": builder["model"], "backbone": args["backbone"], "decoder": args["decoder"],
+    model = BasicModel(args)
+    out["models"][y] = {"model": rec["model"], "backbone": args["backbone"], "decoder": args["decoder"],
                         "state": {k: list(v.shape) for k, v in model.state_dict().items()},
                         "n_params": sum(p.numel() for p in model.parameters())}
 print(json.dumps(out))

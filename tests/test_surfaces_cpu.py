@@ -1,10 +1,18 @@
-"""CPU: the ATen-composed surfaces of megreader_b200.refapi (SURVEY.md §8 A9/A10) reproduce the reference goldens, and —
-where /root/reference is present — carry the reference's exact state-dict keys/shapes, deformable trunk included."""
+"""CPU: the ATen-composed surfaces of megreader_b200.refapi (SURVEY.md §8 A9/A10) reproduce the reference goldens and carry
+the reference's exact state-dict keys/shapes, deformable trunk included."""
+import gzip
+import json
+import os
+
+import numpy as np
 import pytest
 import torch
 
-from oracle import ref_loader
 from tests import surfaces_common as sc
+from tests.weights import east_inputs, fill_state_dict
+
+STATE_GOLD = os.path.join(os.path.dirname(__file__), "golden", "state_dicts_ref.json.gz")
+EAST_GOLD = os.path.join(os.path.dirname(__file__), "golden", "east_ref.npz")
 
 
 def test_backbones_reproduce_reference_golden():
@@ -26,86 +34,71 @@ def test_ctc_conv_head_train_refuses_cpu():
 
 
 def _keys(m):
-    return [(k, tuple(v.shape)) for k, v in m.state_dict().items()]
+    return [[k, list(v.shape)] for k, v in m.state_dict().items()]
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present")
 def test_state_dict_keys_equal_reference():
+    """Keys and shapes equal those of the reference's modules, recorded by `python -m oracle.make_golden state_dicts`."""
     import sys
     import types
-    ref_loader.install()
-    # the reference's DCN python modules import their compiled extension at import time; a placeholder lets the
-    # module *definitions* load so that parameter names can be compared (nothing is executed through it)
-    sys.modules.setdefault("assets.ops.dcn.deform_conv_cuda", types.ModuleType("assets.ops.dcn.deform_conv_cuda"))
-    sys.modules.setdefault("assets.ops.dcn.deform_pool_cuda", types.ModuleType("assets.ops.dcn.deform_pool_cuda"))
-    import backbones as rb
-    import decoders as rd
     import megreader_b200.refapi.backbones as mb
     import megreader_b200.refapi.decoders as md
     import megreader_b200.refapi.backbones.resnet as mres
     from megreader_b200 import dcn as mdcn
-    pairs = [(rb.resnet34(pretrained=False), mb.resnet34(pretrained=False)),
-             (rb.resnet101(pretrained=False), mb.resnet101(pretrained=False)),
-             (rb.Resnet34FPN(resnet_pretrained=False), mb.Resnet34FPN(resnet_pretrained=False)),
-             (rb.resnet50dilated_ppm(inner_channels=128), mb.resnet50dilated_ppm(inner_channels=128)),
-             (rd.AttentionDecoder(64, inner_channels=128, max_size=16, height=2),
-              md.AttentionDecoder(64, inner_channels=128, max_size=16, height=2)),
-             (rd.CTCDecoder(64, inner_channels=96), md.CTCDecoder(64, inner_channels=96)),
-             (rd.EASTDecoder(channels=64), md.EASTDecoder(channels=64))]
-    for r, m in pairs:
-        assert _keys(r) == _keys(m)
+    with gzip.open(STATE_GOLD, "rt") as f:
+        ref = json.load(f)["modules"]
+    mine = {"resnet34": mb.resnet34(pretrained=False), "resnet101": mb.resnet101(pretrained=False),
+            "Resnet34FPN": mb.Resnet34FPN(resnet_pretrained=False),
+            "resnet50dilated_ppm": mb.resnet50dilated_ppm(inner_channels=128),
+            "AttentionDecoder": md.AttentionDecoder(64, inner_channels=128, max_size=16, height=2),
+            "CTCDecoder": md.CTCDecoder(64, inner_channels=96), "EASTDecoder": md.EASTDecoder(channels=64)}
     # deformable trunk: our modules resolve `assets.ops.dcn` lazily; bind it to megreader_b200.dcn for this process
     shim = types.ModuleType("assets.ops.dcn")
     shim.ModulatedDeformConv, shim.DeformConv = mdcn.ModulatedDeformConv, mdcn.DeformConv
-    ref_dcn = rb.deformable_resnet50(pretrained=False)
     saved = sys.modules.get("assets.ops.dcn")
     sys.modules["assets.ops.dcn"] = shim
     try:
-        mine = mres.deformable_resnet50(pretrained=False)
-        mine_v1 = mres.ResNet(mres.BasicBlock, [1, 1, 1, 1], dcn=dict(modulated=False, deformable_groups=2))
+        mine["deformable_resnet50"] = mres.deformable_resnet50(pretrained=False)
+        mine["ResNet_v1_dcn"] = mres.ResNet(mres.BasicBlock, [1, 1, 1, 1], dcn=dict(modulated=False, deformable_groups=2))
     finally:
         if saved is not None:
             sys.modules["assets.ops.dcn"] = saved
-    assert _keys(ref_dcn) == _keys(mine)
-    ref_v1 = rb.resnet.ResNet(rb.resnet.BasicBlock, [1, 1, 1, 1], dcn=dict(modulated=False, deformable_groups=2))
-    assert _keys(ref_v1) == _keys(mine_v1)
-    # zero-initialised offset branch (resnet.py:222-226)
-    for mod in mine.modules():
-        if hasattr(mod, "conv2_offset"):
-            assert float(mod.conv2_offset.weight.abs().max()) == 0.0 and float(mod.conv2_offset.bias.abs().max()) == 0.0
+        else:
+            del sys.modules["assets.ops.dcn"]
     # deformable RoI pooling packs: same fully-connected stacks
-    import assets.ops.dcn.modules.deform_pool as rpool
     from megreader_b200 import deform_pool as mpool
     for cls in ("DeformRoIPoolingPack", "ModulatedDeformRoIPoolingPack"):
-        r = getattr(rpool, cls)(0.5, 3, 8, False, trans_std=0.1, deform_fc_channels=32)
-        m = getattr(mpool, cls)(0.5, 3, 8, False, trans_std=0.1, deform_fc_channels=32)
-        assert _keys(r) == _keys(m)
+        mine[cls] = getattr(mpool, cls)(0.5, 3, 8, False, trans_std=0.1, deform_fc_channels=32)
+    assert sorted(mine) == sorted(ref)
+    for name, m in mine.items():
+        assert _keys(m) == ref[name], name
+    # zero-initialised offset branch (resnet.py:222-226)
+    for mod in mine["deformable_resnet50"].modules():
+        if hasattr(mod, "conv2_offset"):
+            assert float(mod.conv2_offset.weight.abs().max()) == 0.0 and float(mod.conv2_offset.bias.abs().max()) == 0.0
     # dilation surgery moved the same convs (resnet_dilated.py:37-49)
-    rp, mp = rb.resnet50dilated_ppm(), mb.resnet50dilated_ppm()
-    geo = lambda net: [(n, c.stride, c.dilation, c.padding) for n, c in net.named_modules() if isinstance(c, torch.nn.Conv2d)]
-    assert geo(rp) == geo(mp)
+    geo = [[n, list(c.stride), list(c.dilation), list(c.padding)] for n, c in mb.resnet50dilated_ppm().named_modules()
+           if isinstance(c, torch.nn.Conv2d)]
+    with gzip.open(STATE_GOLD, "rt") as f:
+        assert geo == json.load(f)["resnet50dilated_ppm_conv_geometry"]
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="/root/reference not present")
 def test_east_decoder_equals_reference_module():
-    """decoders/east.py:7-60 on CPU: same parameters -> same loss, metrics and predictions (train and eval branches)."""
-    ref_loader.install()
-    import decoders as rd
+    """decoders/east.py:7-60 on CPU: same parameters -> the reference module's loss, metrics and predictions (train and eval
+    branches), recorded by `python -m oracle.make_golden east` with one host thread."""
     import megreader_b200.refapi.decoders as md
-    torch.manual_seed(0)
-    r, m = rd.EASTDecoder(channels=32).train(), md.EASTDecoder(channels=32).train()
-    m.load_state_dict(r.state_dict())
-    x = torch.randn(2, 32, 6, 10)
-    label = {"heatmap": (torch.rand(2, 1, 24, 40) > 0.7).float(), "heatmap_weight": torch.rand(2, 1, 24, 40),
-             "densebox": torch.randn(2, 8, 24, 40) * 50, "densebox_weight": torch.rand(2, 8, 24, 40)}
-    lr, pr, mr_ = r(x, label, None, True)
+    g = np.load(EAST_GOLD)
+    m = fill_state_dict(md.EASTDecoder(channels=32), "east.").train()
+    torch.set_num_threads(1)
+    x, label = east_inputs()
     lm, pm, mm = m(x, label, None, True)
-    torch.testing.assert_close(lm, lr)
-    for k in pr:
-        torch.testing.assert_close(pm[k], pr[k])
-    for k in mr_:
-        torch.testing.assert_close(mm[k], mr_[k])
-    r.eval(); m.eval()
-    pe_r, pe_m = r(x, label, None, False), m(x, label, None, False)
-    for k in pe_r:
-        torch.testing.assert_close(pe_m[k], pe_r[k])
+    torch.testing.assert_close(lm, torch.from_numpy(g["loss"]))
+    for prefix, got in (("pred.", pm), ("metrics.", mm)):
+        assert sorted(prefix + k for k in got) == sorted(k for k in g.files if k.startswith(prefix))
+        for k in got:
+            torch.testing.assert_close(got[k], torch.from_numpy(g[prefix + k]))
+    m.eval()
+    pe_m = m(x, label, None, False)
+    assert sorted("eval." + k for k in pe_m) == sorted(k for k in g.files if k.startswith("eval."))
+    for k in pe_m:
+        torch.testing.assert_close(pe_m[k], torch.from_numpy(g["eval." + k]))

@@ -58,3 +58,14 @@ def surface_inputs():
     for b in range(3):
         targets[b, lengths[b]:] = 0
     return x, x2, feat, targets, lengths
+
+
+def east_inputs():
+    """Seeded inputs of tests/golden/east_ref.npz: a 32-channel feature map and EAST labels at 4x its resolution."""
+    rng = np.random.RandomState(0)
+    x = rng.standard_normal((2, 32, 3, 5)).astype(np.float32)
+    label = {"heatmap": (rng.random_sample((2, 1, 12, 20)) > 0.7).astype(np.float32),
+             "heatmap_weight": rng.random_sample((2, 1, 12, 20)).astype(np.float32),
+             "densebox": (rng.standard_normal((2, 8, 12, 20)) * 50).astype(np.float32),
+             "densebox_weight": rng.random_sample((2, 8, 12, 20)).astype(np.float32)}
+    return torch.from_numpy(x), {k: torch.from_numpy(v) for k, v in label.items()}
