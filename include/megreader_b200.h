@@ -388,6 +388,33 @@ int mr_attn_train_bwd_f32(const float *projected, const float *memory, const flo
                           int E, int V, int S, void *stream);
 int mr_attn_sync_status(const void *sync, void *stream, int *status);
 
+/* ------------------------------------------------------------------------------------------------
+ * DB text detector: SegDetector's probability maps and L1BalanceCELoss (decoders/seg_detector.py:117-147,
+ * decoders/seg_detector_loss.py:157-185, balance_cross_entropy_loss.py:40-54, dice_loss.py:31-42, l1_loss.py:9-11).
+ * fp32 maps, fp32 element math, fp64 sums.  Every map is contiguous.
+ * ---------------------------------------------------------------------------------------------- */
+
+/* b = sigmoid(x_b), t = sigmoid(x_t), tb = 1 / (1 + exp(-k (b - t))), n elements each (accurate expf). */
+int mr_db_maps_fwd_f32(const float *x_b, const float *x_t, int64_t n, float k, float *b, float *t, float *tb, void *stream);
+/* Gradients of the maps above from the saved b, t, tb; any of grad_b / grad_t / grad_tb may be NULL (= zero). */
+int mr_db_maps_bwd_f32(const float *grad_b, const float *grad_t, const float *grad_tb, const float *b, const float *t,
+                       const float *tb, int64_t n, float k, float *grad_xb, float *grad_xt, void *stream);
+/* Bytes of the loss workspace for N samples of HW pixels: 8 per (sample, pixel) plus a fixed ~84 KB. */
+int64_t mr_db_loss_workspace_bytes(int64_t N, int64_t HW);
+/* L1BalanceCELoss forward without host synchronisation.  b, t, tb, gt: (N,1,H,W); mask, thresh_map, thresh_mask: (N,H,W);
+ * gt and mask take values in [0, 1]; 1 <= N <= 256.  Writes out[4] = (loss, bce_loss, thresh_loss (dice), l1_loss) and
+ * keeps in `workspace` what mr_db_loss_bwd_f32 reads (pass the same workspace, unmodified, to the backward). */
+int mr_db_loss_fwd_f32(const float *b, const float *t, const float *tb, const float *gt, const float *mask,
+                       const float *thresh_map, const float *thresh_mask, int64_t N, int64_t HW, float eps,
+                       float l1_scale, float bce_scale, float negative_ratio, float bce_eps, void *workspace,
+                       int64_t workspace_bytes, float *out, void *stream);
+/* Backward for the upstream gradients grad_out[4] of the four outputs (device memory): writes grad_b, grad_t, grad_tb
+ * (N,HW) each.  Among the copies tied at the selection threshold the remainder is split evenly. */
+int mr_db_loss_bwd_f32(const float *grad_out, const float *b, const float *t, const float *gt, const float *mask,
+                       const float *thresh_map, const float *thresh_mask, int64_t N, int64_t HW, float l1_scale,
+                       float bce_scale, const void *workspace, int64_t workspace_bytes, float *grad_b, float *grad_t,
+                       float *grad_tb, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -86,6 +86,11 @@ _SIGS = {
     "mr_dcn_wgrad_fused_f32": [c_p, c_p, c_i64, c_p, c_i64, c_p, c_p, c_f32, c_p, c_i64] + [c_int] * 15 + [c_p],
     "mr_dcn_backward_f32": [c_p, c_p, c_p, c_i64, c_p, c_i64, c_p, c_p, c_p, c_p, c_p, c_i64, c_p, c_i64, c_f32,
                             c_p, c_i64] + [c_int] * 15 + [c_p],
+    "mr_db_maps_fwd_f32": [c_p, c_p, c_i64, c_f32, c_p, c_p, c_p, c_p],
+    "mr_db_maps_bwd_f32": [c_p] * 6 + [c_i64, c_f32, c_p, c_p, c_p],
+    "mr_db_loss_workspace_bytes": [c_i64, c_i64],
+    "mr_db_loss_fwd_f32": [c_p] * 7 + [c_i64, c_i64] + [c_f32] * 5 + [c_p, c_i64, c_p, c_p],
+    "mr_db_loss_bwd_f32": [c_p] * 7 + [c_i64, c_i64, c_f32, c_f32, c_p, c_i64, c_p, c_p, c_p, c_p],
 }
 _RESTYPES = {
     "mr_dcn_workspace_bytes": c_i64,
@@ -93,6 +98,7 @@ _RESTYPES = {
     "mr_dcn_fused_wgrad_workspace_bytes": c_i64,
     "mr_attn_decode_workspace_bytes": c_i64,
     "mr_dcn_fused_backward_workspace_bytes": c_i64,
+    "mr_db_loss_workspace_bytes": c_i64,
     "mr_status_string": ctypes.c_char_p,
     "mr_last_cuda_error": ctypes.c_char_p,
     "mr_launch_count": c_i64,
